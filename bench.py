@@ -56,7 +56,15 @@ def parse_args():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-secondary", action="store_true", help="skip the dragon / glass strong-scaling block")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the image the last one assembled to DIR/image.npy "
+                         "(float32, height x width x 3), to compare two builds on the same inputs")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl != "native":
+        ap.error("--dump-outputs writes what the native arm computed; the reference arm has no such output")
+    return args
 
 
 def workload(name: str, spp_override: int = 0):
@@ -384,6 +392,10 @@ def run_native(args):
         step_ms = sum(step_max)
         kern_ms = sum(kern_max)
         image_mean = float(job.image.mean().item())
+        if args.dump_outputs and rank == 0:  # every rank holds the whole image after the all-gather
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            np.save(os.path.join(args.dump_outputs, "image.npy"),
+                    job.image.view(cfg.height, cfg.width, 3).cpu().numpy())
 
         # ---- e2e: the public call with HOST buffers, copies inside the timed region -----
         e2e = None

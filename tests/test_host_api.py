@@ -255,3 +255,14 @@ def test_bench_arms_share_one_config_and_count_real_cores():
     st = {k: 0 for k in bench.KEYS}
     st.update(segments=10, bvh_node_visits=3, bvh_tri_tests=2, object_tests=4)
     assert bench.algorithmic_bytes(st, 5) == 64 * 4 + 64 * 3 + 52 * 2 + 32 * 10 + 12 * 5
+
+
+@pytest.mark.parametrize("argv", [["--steps", "0"], ["--impl", "reference", "--dump-outputs", "out"]])
+def test_bench_rejects_arguments_it_cannot_honour(argv):
+    """No timed step would leave nothing to time or dump, and the reference arm keeps no image to dump."""
+    import os
+    import subprocess
+    import sys
+    bench = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "bench.py")
+    p = subprocess.run([sys.executable, bench] + argv, capture_output=True, text=True)
+    assert p.returncode == 2 and "error:" in p.stderr and p.stdout == ""

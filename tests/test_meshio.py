@@ -153,20 +153,21 @@ def test_stl_errors():
         api.parse_stl_native(truncated)
 
 
-REF = "/root/reference/examples"
+GOLDEN = os.path.join(os.path.dirname(__file__), "golden")
 
 
-@pytest.mark.skipif(not os.path.exists(REF + "/cylinder.stl"), reason="reference assets only exist in the build container")
 def test_reference_assets_parse():
-    """examples/cylinder.rs and examples/lego.rs inputs: 364 binary facets; the LEGO .obj/.mtl pair cut
-    at every change of `usemtl`."""
-    data = open(REF + "/cylinder.stl", "rb").read()
+    """Inputs of rpt's examples/cylinder.rs and examples/lego.rs: cylinder.stl (364 binary facets), and the
+    LEGO .obj/.mtl pair cut at every change of `usemtl`.  tests/golden keeps cylinder.stl whole; of lego.zip
+    it keeps the .mtl whole and the first 7102 lines of the 21 MB .obj (up to the group `g 123_124`): four
+    material runs, with many repeated `usemtl` of the running material that must not cut."""
+    data = open(os.path.join(GOLDEN, "cylinder.stl"), "rb").read()
     tris = api.parse_stl_native(data)
     assert tris.shape == (364, 18) and np.isfinite(tris).all()
     assert np.array_equal(tris[:, 9:12], tris[:, 15:18])
-    z = zipfile.ZipFile(REF + "/lego.zip")
-    obj = z.read("LEGO.Creator_Plane/LEGO.Creator_Plane.obj")
-    mtl = z.read("LEGO.Creator_Plane/LEGO.Creator_Plane.mtl")
+    z = zipfile.ZipFile(os.path.join(GOLDEN, "lego_plane_head.zip"))
+    obj = z.read("LEGO.Creator_Plane.obj")
+    mtl = z.read("LEGO.Creator_Plane.mtl")
     objects = api.load_obj_with_mtl(io.BytesIO(obj), io.BytesIO(mtl), build=False)
     runs, last = 0, None
     open_faces = False
@@ -181,6 +182,7 @@ def test_reference_assets_parse():
             open_faces, last = False, tok[1]
     runs += open_faces
     assert len(objects) == runs > 1
+    assert [len(o.shape.triangles) for o in objects] == [2, 3696, 416, 64]
     names = api.load_mtl(io.BytesIO(mtl.decode("latin-1").encode()))
     have = {mat_tuple(m) for m in names.values()}
     assert all(mat_tuple(o.mat) in have for o in objects)
